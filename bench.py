@@ -1,8 +1,11 @@
 #!/usr/bin/env python
 """bench.py — CTR samples/sec, forward+backward, batch 65 536 per GPU (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload deepfm|xdeepfm|fibinet|dcn]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload deepfm|xdeepfm|fibinet|dcn] [--dump-outputs DIR]
     python bench.py --impl reference ...        # the reference algorithm on the host cores (oracle port)
+
+With the same arguments every run sees the same seeded weights and batches, so the arrays --dump-outputs writes
+(see dump_outputs) compare two builds of the project output for output.
 
 A step = one pass of the hot path over one synthetic Criteo-shaped batch:
 X[B,39] -> fused gather (+linear, FM) -> interaction + tower -> sigmoid -> BCE(sum) -> backward down
@@ -25,6 +28,7 @@ import time
 
 import torch
 
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from (it may be read-only)
 REPO = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, REPO)
 sys.path.insert(0, os.path.join(REPO, "tests"))
@@ -192,12 +196,12 @@ def host_threads():
 
 
 def load_live_reference():
-    """The UNMODIFIED reference package: baseline/_ref (pip --target install, travels to the GPU box) or the
-    read-only source tree in the build container.  None when neither exists (-> oracle port)."""
+    """The UNMODIFIED reference package: baseline/_ref (scripts/install_reference.sh) or the source tree named by
+    CTR_REFERENCE_ROOT.  None when neither exists (-> oracle port)."""
     sys.path.insert(0, os.path.join(REPO, "tests", "golden"))
     import _ref_loader
-    for root in (os.path.join(REPO, "baseline", "_ref"), "/root/reference"):
-        if os.path.isdir(os.path.join(root, "deepctr_torch")):
+    for root in (os.path.join(REPO, "baseline", "_ref"), _ref_loader.REFERENCE_ROOT):
+        if root and os.path.isdir(os.path.join(root, "deepctr_torch")):
             _ref_loader.REFERENCE_ROOT = root
             try:
                 return _ref_loader.load_reference(), root
@@ -407,6 +411,73 @@ def quick_parity_check(dev):
     return out
 
 
+DUMP_LIMIT_BYTES = 64 * 10**6     # on disk, .npy headers included
+NPY_HEADER_BYTES = 128
+DUMP_TABLE_ROWS = 16384    # most rows of every table whose gradient is written: a fixed seeded sample of the row ids
+
+
+def table_sample_rows(vocab, fixed_bytes, bytes_per_row):
+    """Size of the table row sample: DUMP_TABLE_ROWS, or fewer when the other outputs (``fixed_bytes``) leave less of
+    DUMP_LIMIT_BYTES than DUMP_TABLE_ROWS rows of every table need."""
+    return max(0, min(DUMP_TABLE_ROWS, vocab, (DUMP_LIMIT_BYTES - fixed_bytes) // bytes_per_row))
+
+
+def dump_outputs(out_dir, model, loss, y_pred, pending):
+    """Write what one step hands its caller as ``out_dir/<name>.npy``: ``loss``, ``y_pred``, ``grad.<parameter>`` of
+    every dense parameter and, for every table, the per-unique-row gradients the step leaves for the fused optimizer,
+    as ``grad.<table>.rows`` (the table's gradient at the ids of ``table_sample_ids`` that are below the table's size,
+    zero where the batch does not touch the row) and ``grad.<table>.sum`` (the sum over all its rows, float64).  A
+    table shared by several fields gets the sum of their gradients.  ``table_sample_ids`` is a seeded sample of the
+    largest table's row ids, as many as fit in DUMP_LIMIT_BYTES (at most DUMP_TABLE_ROWS); it depends only on the
+    workload.  ``n_unique_rows`` counts the distinct ids of every id column.  Values are float32, ids and counts
+    float64."""
+    import numpy as np
+    plan = model._plan
+    dev = plan.device
+    names = {id(p): k for k, p in model.named_parameters()}
+    (lease, rg_emb, rg_lin, n_emb), = pending
+    ws = lease.ws
+    n_uniq = ws["n_uniq"].cpu()
+    # table -> (parameter, [(per-unique-row gradients, plan column) of every field that reads it])
+    tables = {}
+    slots = [(p, rg_emb[i], plan.emb_plan_col_host[i]) for i, p in enumerate(plan.emb_params) if i < n_emb] + \
+            [(p, rg_lin[i].unsqueeze(1), plan.lin_plan_col_host[i]) for i, p in enumerate(plan.lin_params)]
+    for p, rg, col in slots:
+        tables.setdefault(names[id(p)], (p, []))[1].append((rg, col))
+    table_ids = set(id(p) for p in plan.emb_params + plan.lin_params)
+    arrays = {"loss": loss.reshape(1), "y_pred": y_pred.reshape(-1), "n_unique_rows": n_uniq.double()}
+    for k, p in model.named_parameters():
+        if id(p) not in table_ids and p.grad is not None:
+            arrays["grad." + k] = p.grad
+    for name, (p, fields) in tables.items():
+        arrays["grad.%s.sum" % name] = sum(rg[:int(n_uniq[col])].double().sum(0) for rg, col in fields)
+    vocab = max(int(p.shape[0]) for p, _ in tables.values())
+    n_files = len(arrays) + 1 + len(tables)          # + table_sample_ids + one grad.<table>.rows per table
+    fixed = sum(a.numel() * a.element_size() for a in arrays.values()) + n_files * NPY_HEADER_BYTES
+    rows = table_sample_rows(vocab, fixed, 8 + sum(4 * int(p.shape[1]) for p, _ in tables.values()))
+    if rows == 0:
+        raise SystemExit("bench.py: --dump-outputs: the dense outputs alone exceed %d bytes" % DUMP_LIMIT_BYTES)
+    sample = np.sort(np.random.RandomState(0).choice(vocab, rows, replace=False))
+    arrays["table_sample_ids"] = torch.from_numpy(sample).double()
+    sample = torch.from_numpy(sample).to(dev)
+    for name, (p, fields) in tables.items():
+        ids = sample[sample < p.shape[0]]
+        out = torch.zeros(len(ids), p.shape[1], device=dev, dtype=torch.float32)
+        for rg, col in fields:
+            n = int(n_uniq[col])
+            pos = torch.full((p.shape[0],), -1, dtype=torch.int64, device=dev)
+            pos[ws["uniq"][col, :n].long()] = torch.arange(n, device=dev)
+            at = pos[ids]
+            out += torch.where((at >= 0).unsqueeze(1), rg[at.clamp_min(0)], 0.0)
+        arrays["grad.%s.rows" % name] = out
+    arrays = {k: v.detach().cpu().numpy() for k, v in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+    written = sum(os.path.getsize(os.path.join(out_dir, k + ".npy")) for k in arrays)
+    assert written <= DUMP_LIMIT_BYTES, written
+
+
 def measure_workload(workload, args, world, rank, dev, steps, warmup, full=True):
     """Time one workload on this process' GPU (all ranks call it together when world > 1).  Returns a dict with the
     device-resident step time, (full) the e2e time, the per-entry-point times of an instrumented eager pass."""
@@ -442,6 +513,8 @@ def measure_workload(workload, args, world, rank, dev, steps, warmup, full=True)
         host_batches.append((X.pin_memory(), y.pin_memory()))
     dev_batches = [(X.to(dev), y.to(dev)) for X, y in host_batches]
     bce = ops.binary_cross_entropy
+    dump_dir = args.dump_outputs if full else None
+    last = {}           # what the last eager step returned, for --dump-outputs
 
     def finish():
         if world > 1:       # dense-grad all-reduce (= barrier for the pushed row gradients) + owner-side combine
@@ -456,6 +529,8 @@ def measure_workload(workload, args, world, rank, dev, steps, warmup, full=True)
         y_pred = model(X)
         loss = bce(y_pred.squeeze(1), y, reduction="sum")
         loss.backward()
+        if dump_dir:
+            last.update(loss=loss, y_pred=y_pred, pending=list(plan.pending))
         finish()
         return loss
 
@@ -545,6 +620,11 @@ def measure_workload(workload, args, world, rank, dev, steps, warmup, full=True)
     out["clocks"] = sampler.stop() if sampler else None
     out["launches"] = timed.launches
     model.check_ids()
+    if dump_dir:            # the outputs of the last timed step, before anything else runs on the model
+        if use_graph:
+            last.update(loss=gstep.loss, y_pred=gstep.y_pred, pending=list(plan.pending))
+        dump_outputs(dump_dir, model, last["loss"], last["y_pred"], last["pending"])
+        last.clear()
     if full:
         pipe = {"primed": False}
         out["e2e_mode"] = "copy-then-step"
@@ -743,9 +823,16 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="issue the step eagerly instead of replaying a CUDA graph")
     ap.add_argument("--allow-eager", action="store_true", help="fall back to the eager step if graph capture fails")
     ap.add_argument("--no-secondary", action="store_true", help="skip the xdeepfm / fibinet / dcn secondary measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (loss, predictions, gradients; table gradients "
+                         "at a fixed sample of rows) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
+    if args.dump_outputs and (args.impl != "b200" or args.gpus != 1 or int(os.environ.get("WORLD_SIZE", "1")) != 1):
+        ap.error("--dump-outputs needs the b200 arm on one GPU")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

@@ -1,7 +1,3 @@
 mkdir -p gpurun_out; rm -rf gpurun_out/*
 echo "== ncu gemm"; timeout -s KILL 400 ncu --set full --clock-control none --import-source on -k regex:gemm_.._kernel -o gpurun_out/gemm_fwd1 python scripts/ncu_gemm.py fwd1 > gpurun_out/ncu_gemm.log 2>&1; echo "ncu exit $?"; ls -la gpurun_out/*.ncu-rep
-echo "== pytest failed subset + new"
-timeout -s KILL 900 python -m pytest tests/test_gpu_gemm.py tests/test_gpu_parity.py tests/test_gpu_round2.py tests/test_gpu_reference_suite.py tests/test_gpu_fit.py -m gpu -q --timeout 800 -p no:cacheprovider --tb=short > gpurun_out/pytest_gpu.log 2>&1
-echo "pytest exit $?"
-grep -E "^(FAILED|ERROR)|passed|failed" gpurun_out/pytest_gpu.log | tail -30 | cut -c1-300
 timeout -s KILL 900 python bench.py --steps 10 --warmup 3 > gpurun_out/bench.log 2>&1; echo "bench exit $?"; tail -c 6000 gpurun_out/bench.log

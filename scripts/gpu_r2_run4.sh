@@ -1,7 +1,6 @@
 mkdir -p gpurun_out; rm -rf gpurun_out/*
 echo "== probe"; timeout -s KILL 120 ./scripts/probe_umma 2>&1 | tee gpurun_out/probe_umma.log | tail -20
 echo "== cin_v2 tests"; CTR_TEST_CIN_V2=1 timeout -s KILL 300 python -m pytest tests/test_gpu_cin_v2.py -m gpu -q --timeout 200 -p no:cacheprovider --tb=short > gpurun_out/pytest_cinv2.log 2>&1; echo "exit $?"; grep -E "^(FAILED|ERROR)|passed|failed|^E  " gpurun_out/pytest_cinv2.log | tail -12 | cut -c1-250
-echo "== reference suite IFM DIFM"; timeout -s KILL 600 python -m pytest tests/test_gpu_reference_suite.py -m gpu -q -k "IFM or DIFM" --timeout 500 -p no:cacheprovider --tb=short > gpurun_out/pytest_ref.log 2>&1; echo "exit $?"; grep -E "^(FAILED|ERROR)|passed|failed" gpurun_out/pytest_ref.log | tail -5 | cut -c1-250
 for v in 0 1; do
   CTR_CIN_V2=$v timeout -s KILL 300 python bench.py --workload xdeepfm --steps 5 --warmup 3 --no-cpu-baseline --no-secondary > gpurun_out/bench_xdeepfm_v2_$v.log 2>&1; echo "bench xdeepfm CIN_V2=$v exit $?"
   grep '^{' gpurun_out/bench_xdeepfm_v2_$v.log | python -c "

@@ -1,12 +1,8 @@
 #!/bin/bash
-# Installs the UNMODIFIED reference into baseline/_ref (git-ignored, travels to the GPU box with the snapshot):
-#   * the package, with pip from a /tmp copy of the read-only tree (--no-deps: torch etc. are already in the image),
-#   * the reference's own test files next to it (baseline/_ref/reftests), so that tests/test_gpu_reference_suite.py
-#     can run them on the GPU with `deepctr_torch` aliased to this repository's package.
+# Installs the UNMODIFIED reference package into baseline/_ref (git-ignored), where `bench.py --impl reference`
+# finds it, with pip from a copy of the read-only tree (--no-deps: torch etc. are already installed).
 set -e
 cd "$(dirname "$0")/.."
 rm -rf /tmp/refcopy && cp -r /root/reference /tmp/refcopy
 python -m pip install --no-index --no-build-isolation --no-deps --find-links /opt/wheelhouse --upgrade --target baseline/_ref /tmp/refcopy
-rm -rf baseline/_ref/reftests && mkdir -p baseline/_ref/reftests
-cp -r /root/reference/tests baseline/_ref/reftests/tests
-ls baseline/_ref baseline/_ref/reftests/tests | head -30
+ls baseline/_ref | head -30

@@ -1,7 +1,7 @@
-"""Import the UNMODIFIED reference (``/root/reference/deepctr_torch``) in the build container.
+"""Import the UNMODIFIED reference (``$CTR_REFERENCE_ROOT/deepctr_torch``).
 
-Only used by ``make_golden.py`` (fixture generation) and by the optional live cross-check test
-that is skipped when ``/root/reference`` is absent (it does not exist on the GPU box).
+Used by ``make_golden.py`` (fixture generation) and by ``bench.py --impl reference``; the tests only read
+the fixtures it produced.
 
 The reference hard-imports ``tensorflow.python.keras.callbacks`` (reference
 ``deepctr_torch/callbacks.py:2-4``, ``models/basemodel.py:22-25``); tensorflow is not installed,
@@ -14,11 +14,11 @@ import os
 import sys
 import types
 
-REFERENCE_ROOT = os.environ.get("CTR_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("CTR_REFERENCE_ROOT", "")
 
 
 def reference_available():
-    return os.path.isdir(os.path.join(REFERENCE_ROOT, "deepctr_torch"))
+    return bool(REFERENCE_ROOT) and os.path.isdir(os.path.join(REFERENCE_ROOT, "deepctr_torch"))
 
 
 def _install_tf_stub():
@@ -50,12 +50,32 @@ def _install_tf_stub():
     leaf.Callback = cb.Callback
 
 
+def _offline_requests():
+    """Stand-in for ``requests`` while the reference is imported: its ``__init__`` asks PyPI for a newer release
+    in a thread (reference ``utils.py:19-44``); this ``get`` fails at once, so no connection is ever opened."""
+    m = types.ModuleType("requests")
+
+    def get(*args, **kwargs):
+        raise ConnectionError("network access is disabled while the reference is loaded")
+    m.get = get
+    m.codes = types.SimpleNamespace(ok=200)
+    return m
+
+
 def load_reference():
     """Return the imported reference package ``deepctr_torch`` (unmodified sources)."""
     if not reference_available():
-        raise RuntimeError("reference tree not found at %s" % REFERENCE_ROOT)
+        raise RuntimeError("reference tree not found at %r (set CTR_REFERENCE_ROOT)" % REFERENCE_ROOT)
     _install_tf_stub()
     if REFERENCE_ROOT not in sys.path:
         sys.path.insert(0, REFERENCE_ROOT)
-    import deepctr_torch  # noqa: E402  (the reference; prints one PyPI notice when offline)
+    saved = sys.modules.get("requests")
+    sys.modules["requests"] = _offline_requests()
+    try:
+        import deepctr_torch  # noqa: E402  (the reference; prints one "check the latest version" notice)
+    finally:
+        if saved is None:
+            del sys.modules["requests"]
+        else:
+            sys.modules["requests"] = saved
     return deepctr_torch

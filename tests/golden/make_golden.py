@@ -1,8 +1,10 @@
 """Generate golden input/output vectors by running the UNMODIFIED reference on CPU.
 
-Run in the build container (needs ``/root/reference``):
+Needs a checkout of the reference project:
 
-    python tests/golden/make_golden.py
+    CTR_REFERENCE_ROOT=<reference checkout> python tests/golden/make_golden.py
+
+(``--round2`` skips the round-1 fixtures; ``--round2 --only=<case>`` or ``--round2 --only=dice`` writes one file.)
 
 Writes ``tests/golden/<case>.npz`` (+ the model description as a JSON string inside each file).
 Each model case records: ``X``, ``y``, every ``state_dict`` tensor (``state/<key>``), the
@@ -32,7 +34,7 @@ from oracle import ctr_oracle as O  # noqa: E402
 ref = load_reference()
 from deepctr_torch.inputs import SparseFeat, DenseFeat, VarLenSparseFeat  # noqa: E402
 from deepctr_torch import models as RM  # noqa: E402
-from deepctr_torch.layers import interaction as RI, core as RC  # noqa: E402
+from deepctr_torch.layers import activation as RA, interaction as RI, core as RC  # noqa: E402
 
 
 def to_ref_columns(cols):
@@ -336,6 +338,31 @@ def fit_case(optimizer="adam", l2=1e-5, fname="fit_criteo_sample"):
     print("wrote %s.npz history:" % fname, hist.history)
 
 
+def dice_case():
+    """The reference Dice (layers/activation.py) on the inputs of tests/test_activation.py, in training then in
+    evaluation mode, and the state_dict keys of a Dice tower (layers/core.py DNN)."""
+    out = {}
+    for dim, shape in ((2, (64, 8)), (3, (16, 5, 8))):
+        torch.manual_seed(0)
+        d = RA.Dice(shape[-1], dim)
+        with torch.no_grad():
+            d.alpha.copy_(torch.randn_like(d.alpha))
+            d.bn.weight.copy_(torch.rand(shape[-1]) + 0.5)
+            d.bn.bias.copy_(torch.randn(shape[-1]) * 0.1)
+        x = torch.randn(*shape)
+        tag = "dim%d" % dim
+        out[tag + "/x"] = x.numpy()
+        for k, v in d.state_dict().items():
+            out[tag + "/state/" + k] = v.detach().clone().numpy()     # before the forwards update the BN buffers
+        for mode in (True, False):
+            d.train(mode)
+            out[tag + ("/y_train" if mode else "/y_eval")] = d(x).detach().numpy()
+    keys = list(RC.DNN(10, [8, 4], activation="dice", dice_dim=2).state_dict().keys())
+    out["dnn_dice_keys"] = json.dumps(keys)
+    np.savez_compressed(os.path.join(HERE, "dice.npz"), **out)
+    print("wrote dice.npz (%d arrays)" % len(out))
+
+
 if __name__ == "__main__":
     torch.set_num_threads(4)
     only_new = "--round2" in sys.argv          # keep the round-1 files byte-identical
@@ -348,9 +375,12 @@ if __name__ == "__main__":
     for case in extra_cases():
         if not only or case[0] in only:
             run_model_case(*case)
+    if "dice" in only:
+        dice_case()
     if only:
         sys.exit(0)
     extra_layer_cases()
     # the fused row-wise optimizer equals the dense torch optimizer for sgd / adagrad at l2 = 0
     fit_case("sgd", 0.0, "fit_sgd_l2zero")
     fit_case("adagrad", 0.0, "fit_adagrad_l2zero")
+    dice_case()

@@ -9,7 +9,7 @@ import torch
 GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 MODEL_CASES = sorted(os.path.basename(p)[:-4] for p in glob.glob(os.path.join(GOLDEN_DIR, "*.npz"))
-                     if not os.path.basename(p).startswith(("layers", "fit_")))
+                     if not os.path.basename(p).startswith(("layers", "fit_", "dice")))
 
 
 def load_case(name):
